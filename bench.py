@@ -6,6 +6,7 @@ backward + gradient all-reduce + AdamW), bs=1024 per GPU, bf16 tensor-core math,
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W                     # ours, N GPUs (weak scaling)
     python bench.py --impl reference --steps 3 --warmup 1          # reference arm: CPU fp32 port of the reference path
+    python bench.py --steps 5 --warmup 3 --dump-outputs DIR        # also write the last timed step's outputs as DIR/*.npy
 
 Prints ONE JSON line (rank 0).  See DESIGN.md §Measurement for every field.
 """
@@ -53,7 +54,12 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true",
                     help="skip the info-only same-box torch eager bf16-autocast leg of the default run")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def measured_peaks():
@@ -277,6 +283,36 @@ class ClockSampler:
 
 
 # ----------------------------------------------------------------------------------------------------------------
+# outputs of the timed path, for comparing two builds (the inputs and the initial weights are seeded)
+# ----------------------------------------------------------------------------------------------------------------
+def dump_outputs(dirname, model, loss_mod, loss, n_sample=1 << 23):
+    """Writes what the last timed step computed, as its caller receives it, in float32: loss.npy (the step's loss),
+    logit_scale.npy (the updated temperature parameter) and weights.npy, the updated weights at a fixed seeded sample of
+    n_sample positions of the model's parameters in named_parameters() order (~600 MB in full, 32 MB as sampled).  The
+    parameters' .grad views hold nothing by then: the fused AdamW step clears them.  The training step is not yet
+    bit-reproducible: split-K GEMMs (TMA reduce-add) and the LayerNorm / bias / embedding / logit-scale gradient
+    reductions accumulate with fp32 atomics, and AdamW turns last-bit differences in near-zero gradients into weight
+    differences of up to 2 * lr, so two runs of one build differ by up to ~1e-3 in the weights."""
+    import numpy as np
+    import torch
+
+    params = [p for _, p in model.named_parameters()]
+    sizes = torch.tensor([p.numel() for p in params])
+    ends = sizes.cumsum(0)
+    pos = torch.randint(0, int(ends[-1]), (n_sample,), generator=torch.Generator().manual_seed(0)).sort().values
+    cut = torch.searchsorted(pos, ends).tolist()   # pos[cut[i - 1]:cut[i]] fall into params[i]
+    weights, lo = [], 0
+    for p, hi, start in zip(params, cut, (ends - sizes).tolist()):
+        weights.append(p.detach().reshape(-1)[(pos[lo:hi] - start).to(p.device)])
+        lo = hi
+    out = {"loss": loss.detach().reshape(1), "logit_scale": loss_mod.logit_scale.detach().reshape(1),
+           "weights": torch.cat(weights)}
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), t.float().cpu().numpy())
+
+
+# ----------------------------------------------------------------------------------------------------------------
 # our arm
 # ----------------------------------------------------------------------------------------------------------------
 def run_ours(args):
@@ -358,6 +394,8 @@ def run_ours(args):
     ms_dev = max_over_ranks(e0.elapsed_time(e1) / args.steps)
     launches = (_lib.LAUNCHES - launches0) // args.steps
     final_loss = float(loss.item())
+    if args.dump_outputs and rank == 0:   # before the steps below change the weights again
+        dump_outputs(args.dump_outputs, model, loss_mod, loss)
 
     # ---- per-kernel-family breakdown: INSTR_STEPS more steps with every GEMM / attention / LayerNorm launch bracketed
     # by CUDA events on the launching stream (kept out of the region above: ~1000 event records per step) ----

@@ -9,6 +9,8 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+import clip_cases as CC  # noqa: E402
 from multimodal_b200 import ops  # noqa: E402
 from oracle import clip_oracle as O  # noqa: E402
 
@@ -95,7 +97,7 @@ def e2e_small():
     gold = torch.load(os.path.join(ROOT, "tests/golden/clip_golden.pt"), map_location="cpu", weights_only=False)["clip_small"]
     m = CLIP(CLIPViTEncoder(64, 16, 64, 128, 2, 2),
              CLIPTextEncoder(embedding_dim=64, vocab_size=512, width=128, dim_feedforward=512, heads=2, layers=2))
-    m.load_state_dict(gold["state_dict"])
+    m.load_state_dict(CC.small_state_dict(gold))
     m = m.to(dev).train()
     loss_mod = ContrastiveLossWithTemperature().to(dev)
     img, txt = gold["image"].to(dev), gold["text"].to(dev)

@@ -33,7 +33,7 @@ def main():
               text_masked=inp["text_masked"], skip_unmasked_mm_encoder=False)
         got = FC.flatten_output(o)
         for k, ref in g["outputs"].items():
-            err = (got[k] - ref).abs().max().item()
+            err = (FC.golden_view(got[k]) - ref).abs().max().item()
             log(f"{name} {k}: abs_err={err:.3e} ref_absmax={ref.abs().max().item():.3e} rel={err / ref.abs().max().item():.3e}")
     # ---- config 3 timing
     B = int(os.environ.get("FLAVA_BS", "256"))

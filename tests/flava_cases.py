@@ -73,3 +73,14 @@ def flatten_output(out) -> dict:
     res["projected_image_embeddings"] = out.projected_image_embeddings
     res["projected_text_embeddings"] = out.projected_text_embeddings
     return {k: v.detach().float().cpu().clone() for k, v in res.items() if v is not None}
+
+
+GOLDEN_TOKENS = 8
+
+
+def golden_view(t: torch.Tensor) -> torch.Tensor:
+    """The part of an output the fixture stores, so that it stays small: of a [B, S, D] sequence output with more than
+    GOLDEN_TOKENS positions, the first, the last and evenly spaced positions between them; anything else whole."""
+    if t.dim() != 3 or t.shape[1] <= GOLDEN_TOKENS:
+        return t
+    return t[:, torch.linspace(0, t.shape[1] - 1, GOLDEN_TOKENS).round().long().to(t.device)]

@@ -1,13 +1,11 @@
-"""Generates tests/golden/*.pt by running the UNMODIFIED reference (imported from /root/reference, which exists only
-in the build container) on small deterministic inputs.  Committed together with its outputs; the GPU box only ever
-reads the .pt files.
+"""Generates tests/golden/clip_golden.pt by running the UNMODIFIED reference (a TorchMultimodal checkout, given as the
+argument) on small deterministic inputs.  Committed together with its outputs; the tests only ever read the .pt file.
 
-    PYTHONPATH=oracle/iopath_shim:/root/reference python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <path to the TorchMultimodal checkout>
 
-Cases (kept tiny so the fixtures stay small; weights are regenerated from seeds, only inputs/outputs are stored):
-  clip_small : CLIP(CLIPViTEncoder(64, 16, 64, 128, 2, 2), CLIPTextEncoder(64, vocab=512, width=128, ff=512, heads=2, layers=2))
-               B=4, image 64x64, reference init under torch.manual_seed(0); fp32 forward, loss, and all gradients
-               (stored as per-tensor float64 sums + a few raw tensors).
+Cases (kept tiny so the fixture stays small; weights are regenerated from seeds, only inputs/outputs are stored):
+  clip_small : tests/clip_cases.py's small CLIP (64x64 images, width 128, 2 layers per tower), B=4; fp32 forward, loss,
+               and all gradients (per-tensor float64 sums + a few raw tensors), and per-tensor checksums of the weights.
   clip_b16_b2: clip_vit_b16() under torch.manual_seed(0), B=2 synthetic batch; embeddings + loss only.
 """
 import math
@@ -19,8 +17,9 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, os.path.join(ROOT, "oracle", "iopath_shim"))
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.path.abspath(sys.argv[1]))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 from torchmultimodal.models.clip.image_encoder import CLIPViTEncoder  # noqa: E402
 from torchmultimodal.models.clip.model import CLIP, clip_vit_b16  # noqa: E402
@@ -30,25 +29,15 @@ from torchmultimodal.modules.losses.contrastive_loss_with_temperature import (  
     contrastive_loss_with_temperature,
 )
 
+import clip_cases as CC  # noqa: E402
 from oracle import clip_oracle as O  # noqa: E402
-
-
-def small_model():
-    torch.manual_seed(0)
-    enc_a = CLIPViTEncoder(embedding_dim=64, patch_size=16, image_size=64, width=128, heads=2, layers=2)
-    enc_b = CLIPTextEncoder(embedding_dim=64, vocab_size=512, width=128, dim_feedforward=512, heads=2, layers=2)
-    return CLIP(enc_a, enc_b)
 
 
 def main():
     torch.set_num_threads(8)
     out = {}
     # ---------------- clip_small: forward + loss + grads ----------------
-    m = small_model().train()
-    with torch.no_grad():  # break the "all layers identical" symmetry of nn.TransformerEncoder's deepcopy init
-        g = torch.Generator().manual_seed(7)
-        for p in m.parameters():
-            p.add_(0.02 * torch.randn(p.shape, generator=g))
+    m = CC.build_small(CLIP, CLIPViTEncoder, CLIPTextEncoder).train()
     img, txt = O.synthetic_batch(4, image_size=64, vocab=512)
     loss_mod = ContrastiveLossWithTemperature()
     o = m(img, txt)
@@ -56,7 +45,7 @@ def main():
     res.loss.backward()
     out["clip_small"] = {
         "image": img, "text": txt,
-        "state_dict": {k: v.clone() for k, v in m.state_dict().items()},
+        "state_dict_checksum": CC.state_dict_checksum(m.state_dict()),
         "emb_a": o.embeddings_a.detach().clone(), "emb_b": o.embeddings_b.detach().clone(),
         "loss": res.loss.detach().clone(), "logits_a": res.logits_a.detach().clone(),
         "logits_b": res.logits_b.detach().clone(),

@@ -12,6 +12,7 @@ import math
 import pytest
 import torch
 
+import clip_cases as CC
 from oracle import clip_oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -310,7 +311,7 @@ def test_clip_small_against_reference_golden(dev, golden):
         ContrastiveLossWithTemperature, contrastive_loss_with_temperature)
 
     g = golden["clip_small"]
-    m = _small_clip(dev, g["state_dict"])
+    m = _small_clip(dev, CC.small_state_dict(g))
     loss_mod = ContrastiveLossWithTemperature().to(dev)
     out = m(g["image"].to(dev), g["text"].to(dev))
     assert (out.embeddings_a.cpu() - g["emb_a"]).abs().max() < 3e-3

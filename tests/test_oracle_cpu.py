@@ -6,12 +6,13 @@ import math
 import pytest
 import torch
 
+import clip_cases as CC
 from oracle import clip_oracle as O
 
 
 def test_oracle_small_forward_and_grads_match_reference_golden(golden):
     g = golden["clip_small"]
-    sd = {k: v.clone().requires_grad_(v.is_floating_point()) for k, v in g["state_dict"].items()}
+    sd = {k: v.clone().requires_grad_(v.is_floating_point()) for k, v in CC.small_state_dict(g).items()}
     scale = torch.tensor(math.log(1 / 0.07), requires_grad=True)
     a, b = O.clip_forward(g["image"], g["text"], sd, img_heads=2, txt_heads=2)
     loss, la, lb, _, _ = O.contrastive_loss(a, b, scale)
@@ -55,9 +56,10 @@ def test_oracle_b16_forward_matches_reference_golden_and_init_mirror(golden):
 def test_fused_timing_variant_matches_oracle(golden):
     """bench.py's CPU arm uses oracle.clip_forward_fused (library-fused ops); it must be the same function."""
     g = golden["clip_small"]
+    sd = CC.small_state_dict(g)
     with torch.no_grad():
-        a, b = O.clip_forward(g["image"], g["text"], g["state_dict"], 2, 2)
-        af, bf = O.clip_forward_fused(g["image"], g["text"], g["state_dict"], 2, 2)
+        a, b = O.clip_forward(g["image"], g["text"], sd, 2, 2)
+        af, bf = O.clip_forward_fused(g["image"], g["text"], sd, 2, 2)
     torch.testing.assert_close(af, a, rtol=0, atol=2e-6)
     torch.testing.assert_close(bf, b, rtol=0, atol=2e-6)
 
